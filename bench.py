@@ -277,6 +277,8 @@ def run_native(args, w, rank, world, local_rank):
     ms_dev, launches, wall_dev, per_step = one_pass(dev, True, sampler)
     worst_dev = dict(one_pass.worst_step)
     ms_e2e, _, wall_e2e, per_step_e2e = one_pass(pin, False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(slam, args.dump_outputs)
     surfels = slam.getMap().size()
     gt = np.linalg.inv(synth.trajectory(1)[0]) @ synth.trajectory(n_frames)[-1]
     drift = float(np.linalg.norm(slam.getCurrentPose()[:3, 3] - gt[:3, 3]))
@@ -409,6 +411,41 @@ def run_native(args, w, rank, world, local_rank):
     return out
 
 
+DUMP_SURFELS = 1 << 17  # at most this many surfel records (a fixed, seeded sample of the map) go to surfels.npy
+
+
+def dump_outputs(slam, out_dir):
+    """what a caller of processScan receives after the last timed step, as DIR/<name>.npy (float32 / float64, < 64 MB):
+    the pose, the ICP statistics, the surfel map (count + sampled records) and the current data / model frames"""
+    os.makedirs(out_dir, exist_ok=True)
+    st = slam.getStatistics()
+    surf = slam.getMap().getAllSurfels()
+    n = surf.shape[0]
+    idx = np.arange(n) if n <= DUMP_SURFELS else np.sort(np.random.default_rng(0).choice(n, DUMP_SURFELS, replace=False))
+    out = {"pose": slam.getCurrentPose(),
+           "icp_statistics": np.array([st[k] for k in ("num_iterations", "F", "inlier", "outlier", "invalid",
+                                                       "inlier_residual", "track_loss")], np.float64),
+           "surfel_count": np.array([n], np.float64),
+           "surfel_sample_index": idx.astype(np.float64),
+           "surfels": np.stack([surf[f][idx].astype(np.float32) for f in surf.dtype.names], 1)}
+    for name, frame in (("current_frame", slam.getCurrentFrame()), ("current_model_frame", slam.getCurrentModelFrame())):
+        for part, a in zip(("vertex", "normal", "semantic"), frame.maps()):
+            out["%s_%s" % (name, part)] = a
+    for k, v in list(out.items()):
+        # Every file holds finite numbers only. A non-finite element is written as 0, and <name>_nonfinite.npy lists it
+        # as (flat index, 1 = NaN / 2 = +inf / 3 = -inf). Such elements are part of the result: the reference's
+        # slerp (update_surfels.vert:113-124) divides by sin(0) when a surfel's normal equals the measured one, which
+        # leaves that surfel's normal NaN.
+        bad = np.flatnonzero(~np.isfinite(v))
+        if bad.size:
+            flat = v.reshape(-1)
+            code = np.where(np.isnan(flat[bad]), 1, np.where(flat[bad] > 0, 2, 3))
+            out[k + "_nonfinite"] = np.stack([bad, code], 1).astype(np.float64)
+            out[k] = np.where(np.isfinite(v), v, 0).astype(v.dtype)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 class StripedGuard(threading.Thread):
     """deadline for the optional `striped` record of the N > 1 runs (see run_native)"""
 
@@ -536,8 +573,7 @@ def cpu_baseline(w, scans, budget_s=15.0, max_frames=None):
             "sample": "first %d scans of the same synthetic sequence (map grows from empty), oracle/ C port, %d OpenMP "
                       "threads = physical cores of one socket" % (n, threads),
             "single_thread": {"value": round(single, 3), "unit": "scans/s", "cores": 1, "sample": "first %d scans" % n1},
-            "seconds": round(dt, 2), "host_cpus": os.cpu_count(),
-            "reference_itself": reference_itself_sample(w, scans, budget_s=8.0, max_frames=4)}
+            "seconds": round(dt, 2), "host_cpus": os.cpu_count()}
 
 
 def reference_itself_sample(w, scans, budget_s=12.0, max_frames=6):
@@ -680,6 +716,9 @@ def main():
     ap.add_argument("--no-prefetch", dest="prefetch", action="store_false",
                     help="e2e pass: do not stage scan i+1 on the copy stream while scan i is processed (sb_prefetch_scan); "
                          "with or without it every copy is inside the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (pose, statistics, surfels, frames) as "
+                         "DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=15.0)

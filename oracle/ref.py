@@ -344,6 +344,10 @@ class Full:
         if getattr(self, "h", None):
             self.L.reffull_destroy(self.h); self.h = None
 
+    def zero_stale_tail(self, on):
+        """process-wide: whether the next scans read 0 (not the previous scan's values) past the labels just uploaded"""
+        self.L.reffull_zero_stale_tail(C.c_int(1 if on else 0))
+
     def _check(self, r):
         err = self.L.reffull_error(self.h).decode()
         if r != 0 or err:

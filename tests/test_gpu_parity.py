@@ -399,9 +399,7 @@ def test_fused_peer_exchange_in_one_gpu_loop_back():
 def test_cuda_equals_reference_shaders_directly():
     """the CUDA path against oracle/_ref (the reference's own shader text on a software GL, pinned built-ins): images,
     index map, surfels and their order, bit for bit -- no hand-written oracle in between"""
-    from oracle import ref as R
-    if not R.available():
-        pytest.skip("oracle/_ref not shipped")
+    from reference_replay import R   # the reference's outputs, replayed from tests/golden/reference_calls/
     po, pp = both_params(**sized(900))
     ctx = api.Context(pp)
     sc, poses = scans(900, n=3, semantic=True)

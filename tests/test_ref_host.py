@@ -6,7 +6,10 @@ compiled where they lie under /root/reference (oracle/ref_harness/Makefile) agai
 What is compared with it: the oracle (oracle/orc_core.c), the host-side math the product exports through the C ABI
 (sb_se3_exp, sb_se3_log, sb_gn_step -- pure host functions, callable without a GPU), semantic_suma_b200/kitti.py and
 include/suma_b200_io.hpp. Tolerances, not bits: the operation order inside Eigen's products is Eigen's; the stand-in uses
-left-to-right IEEE. Decisions (iteration counts, history lengths, segment selection) must be equal."""
+left-to-right IEEE. Decisions (iteration counts, history lengths, segment selection) must be equal.
+
+What the reference returned is replayed from tests/golden/reference_calls/ (tests/reference_replay.py), so these
+comparisons need neither the reference nor oracle/_ref."""
 import ctypes as C
 import os
 import shutil
@@ -16,13 +19,12 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from oracle import ref as R
+from oracle import ref
 from semantic_suma_b200 import api, kitti, synth
 from helpers import scans, sized
+from reference_replay import R
 
-pytestmark = pytest.mark.skipif(not R.host_available(), reason="oracle/_ref host library not built and /root/reference absent")
-
-REF_XML = os.path.join(R.REFERENCE, "config", "default.xml")
+REF_XML = os.path.join(ref.REFERENCE, "config", "default.xml")
 
 
 def _dp(a):
@@ -189,7 +191,6 @@ def test_icp_minimize_equals_the_reference_loop_on_real_frames():
 
 
 # ---------------------------------------------------------------------------------------------- parameters
-@pytest.mark.skipif(not os.path.exists(REF_XML), reason="/root/reference absent (GPU box)")
 def test_default_xml_through_the_reference_parser():
     """config/default.xml read by the reference's own rv::parseXmlFile: every key of the committed fixture
     (tests/golden/reference_default_xml.json, made by a Python XML parser) has the same value, and our defaults follow"""
@@ -322,7 +323,8 @@ def test_cpp_io_header_equals_the_reference_devkit(tmp_path):
     kitti.save_poses(tmp_path / "gt.txt", gt)
     kitti.save_poses(tmp_path / "est.txt", est)
     out = subprocess.check_output([exe, str(tmp_path / "gt.txt"), str(tmp_path / "est.txt")], text=True).split("\n")
-    rows = R.kitti_sequence_errors(R.kitti_load_poses(tmp_path / "gt.txt"), R.kitti_load_poses(tmp_path / "est.txt"))
+    rows = R.computed(lambda: R.kitti_sequence_errors(R.kitti_load_poses(tmp_path / "gt.txt"),
+                                                      R.kitti_load_poses(tmp_path / "est.txt")))
     assert int(out[0]) == rows.shape[0] > 0
     for line, r in zip(out[1:], rows):
         v = [float(x) for x in line.split()]

@@ -10,7 +10,9 @@ and driven by a minimal software GL that issues the draw calls of Preprocessing.
   precise  the same built-ins in fp64/libm: an independent GL. Decisions (validity, labels, counters, surfel counts) may
            differ only where a value sits within rounding of a threshold; floats agree to the stated tolerances.
 
-Both builds were made from the reference's files where they lie; nothing of the reference is in the repository.
+Both builds were made from the reference's files where they lie; nothing of the reference is in the repository. What
+they returned is replayed from tests/golden/reference_calls/ (tests/reference_replay.py), so these comparisons need
+neither the reference nor oracle/_ref.
 """
 import os
 
@@ -18,10 +20,9 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from oracle import ref as R
+from oracle import ref
 from helpers import assert_bits_equal, bits, scans, sized, surfel_fields_equal
-
-pytestmark = pytest.mark.skipif(not R.available(), reason="oracle/_ref not built and /root/reference absent")
+from reference_replay import R
 
 MOVABLE = (10, 11, 13, 15, 18, 20, 30, 31, 32)
 
@@ -33,18 +34,21 @@ def _frames_equal(a, b, what):
 
 def test_ref_is_generated_from_the_reference_sources():
     """the manifest names every hot-path shader with the hash of the file it was generated from"""
-    man = open(os.path.join(os.path.dirname(R.lib_path("pinned")), "gen", "MANIFEST.txt")).read()
+    manifest = os.path.join(os.path.dirname(ref.lib_path("pinned")), "gen", "MANIFEST.txt")
+    if not os.path.exists(manifest):
+        pytest.skip("oracle/_ref not built (it is built from a checkout of the reference)")
+    man = open(manifest).read()
     for sh in ("gen_vertexmap.vert", "gen_normalmap.frag", "floodfill.frag", "Frame2Model_jacobians.geom",
                "render_surfels.geom", "render_surfels.frag", "render_compose.frag", "gen_indexmap.vert",
                "init_radiusConf.vert", "update_surfels.vert", "update_surfels.geom", "gen_surfels.geom",
                "copy_surfels.vert"):
         assert "shader/%s@" % sh in man, sh
-    if R.have_reference():
+    if ref.have_reference():
         import hashlib
         for line in man.splitlines():
             for item in line.split("<- ")[1].split(", "):
                 rel, h = item.split("@")
-                src = open(os.path.join(R.REFERENCE, "src", rel)).read()
+                src = open(os.path.join(ref.REFERENCE, "src", rel)).read()
                 assert hashlib.sha256(src.encode()).hexdigest()[:16] == h, rel
 
 
@@ -105,11 +109,13 @@ def test_preprocess_against_an_independent_gl():
     p = O.default_params(**sized(900))
     sc, _ = scans(900, n=1, semantic=True)
     a = O.preprocess(p, *sc[0], timestamp=20)
-    b = R.preprocess(p, *sc[0], timestamp=20, mode="precise")
+    with R.sampled(1):
+        b = R.preprocess(p, *sc[0], timestamp=20, mode="precise")
     assert_bits_equal(a[0], b[0], "vertex map")
     assert_bits_equal(a[2], b[2], "semantic map")
     assert_bits_equal(a[1][..., 3], b[1][..., 3], "normal validity")
-    assert np.nanmax(np.abs(a[1] - b[1])) < 5e-5
+    idx, normals = R.sample(b[1])   # a fixed, seeded sample of the pixels
+    assert np.nanmax(np.abs(a[1].reshape(-1, 4)[idx] - normals)) < 5e-5
 
 
 # ------------------------------------------------------------------------------------------------- K5
@@ -174,9 +180,9 @@ def _maps(p, mode="pinned"):
 def _check_update(om, rm, what):
     io, ro, go, nuo, nno = om.update_debug()
     ir, rr, gr, nur, nnr = rm.update_debug()
-    assert np.array_equal(io, ir), what + ": index map"
+    assert_bits_equal(io, ir, what + ": index map")
     assert_bits_equal(ro, rr, what + ": radius map")
-    assert np.array_equal(go, gr), what + ": integrated flags"
+    assert_bits_equal(go, gr, what + ": integrated flags")
     assert (nuo, nno) == (nur, nnr), what + ": transform feedback counts"
     surfel_fields_equal(om.download(), rm.download(), what + ": surfels")
 
@@ -265,8 +271,11 @@ def test_map_against_an_independent_gl():
     om, rm = _maps(p, "precise")
     for t in range(3):
         data = O.preprocess(p, *sc[t], timestamp=t)
-        fo, fr = om.render(poses[t], poses[t], 0.0), rm.render(poses[t], poses[t], 0.0)
-        same = np.all(np.abs(fo[0] - fr[0]) < 1e-3, axis=2)
+        fo = om.render(poses[t], poses[t], 0.0)
+        with R.sampled(0):
+            fr = rm.render(poses[t], poses[t], 0.0)
+        idx, vertices = R.sample(fr[0])   # a fixed, seeded sample of the pixels
+        same = np.all(np.abs(fo[0].reshape(-1, 4)[idx] - vertices) < 1e-3, axis=1)
         if t:
             assert same.mean() > 0.97           # the winner of a pixel changes only at depth ties / disc borders
         om.update(poses[t], data); rm.update(poses[t], data)
